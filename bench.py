@@ -6,6 +6,7 @@
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the UNMODIFIED reference's CPU forward on the host cores (oracle/_ref)
     python bench.py --workload cfg3|cfg4|cfg5 # the other BASELINE.json configs (decode, 64K prefill, EP fwd+bwd unit)
+    python bench.py --dump-outputs DIR        # also write what the last timed step computed as DIR/<name>.npy (float32)
 
 Default workload (BASELINE.json configs[1], SURVEY.md §8d cfg 2): random-init Aria-25.3B (seed 0), one synthetic
 980x980 image (4900 patches -> 256 image tokens) + 512 random text tokens => T = 768 prefill tokens,
@@ -21,6 +22,10 @@ Printed JSON (rank 0, one line):
   roofline     the DOMINANT kernel of that table (largest share of the step), in the contract's format
   cpu_baseline the unmodified reference (kind "reference"; oracle port if it is not staged) timed on the host cores on a
                bounded sample of the same workload
+--dump-outputs DIR writes, after the timed steps, the arrays the timed path returned in its last step (rank 0): the logits for
+cfg2/3/4; dx and every weight gradient for cfg5.  Every input is seeded, so two builds run with the same arguments can be
+compared array by array.  An array of more than DUMP_BUDGET / 4 / (number of arrays) elements is replaced by a fixed, seeded
+sample of its elements (same positions in every run), so that a dump stays within DUMP_BUDGET bytes.
 Multi-GPU (--gpus N > 1): every rank prefills its own request (weak scaling) and the routed experts of every MoE layer are
 SHARDED over the ranks — token rows travel over NVLink peer memory (aria_b200/expert_parallel.py); `--multi replicas` runs N
 independent replicas instead (no data-path collective).  See DESIGN.md §5.
@@ -40,6 +45,7 @@ sys.path.insert(0, ROOT)
 
 T_TEXT, T_IMG = 512, 256
 T_TOTAL = T_TEXT + T_IMG
+DUMP_BUDGET = 64 << 20      # bytes written by --dump-outputs
 METRICS = {
     "cfg2": "Aria-25.3B bf16 prefill tokens/sec",
     "cfg3": "Aria-25.3B bf16 decode tokens/sec (batch 32, 2K KV cache)",
@@ -494,6 +500,9 @@ class Cfg2Prefill:
         self.logits_host.copy_(out, non_blocking=False)        # D2H read of the step's result (synchronises)
         return self.logits_host
 
+    def outputs(self, out):
+        return {"logits": out}
+
     def parallelism(self):
         if self.world == 1:
             return "single GPU"
@@ -526,8 +535,9 @@ class Cfg3Decode:
         init_random_(self.model, 0)
         self.n_params = sum(p.numel() for p in self.model.parameters())
         self.cache = self.model.language_model.new_cache(B, self.Tkv + 8, dev)
+        gkv = torch.Generator(device=dev).manual_seed(78 + rank)
         for t in self.cache.k + self.cache.v:
-            t.normal_()
+            t.normal_(generator=gkv)
         g = torch.Generator().manual_seed(77 + rank)
         self.ids_host = torch.randint(10, 100352, (B, 1), generator=g).pin_memory()
         self.ids = self.ids_host.to(dev)
@@ -559,6 +569,9 @@ class Cfg3Decode:
         self.graph.replay()
         self.logits_host.copy_(self.out)
         return self.logits_host
+
+    def outputs(self, out):
+        return {"logits": out}
 
     def parallelism(self):
         return "single GPU" if self.world == 1 else f"replicas x{self.world} (no data-path collective)"
@@ -600,6 +613,9 @@ class Cfg4LongPrefill:
         out = self.model(self.ids_host, self.pv_host, None, num_logits_to_keep=1).logits
         self.logits_host.copy_(out)
         return self.logits_host
+
+    def outputs(self, out):
+        return {"logits": out}
 
     def parallelism(self):
         return "single GPU" if self.world == 1 else f"replicas x{self.world} (no data-path collective)"
@@ -656,6 +672,9 @@ class Cfg5EpTrain:
         self.dx_host.copy_(self.step_eager())
         return self.dx_host
 
+    def outputs(self, out):
+        return {"dx": out, **{"d_" + n.replace(".", "_"): p.grad for n, p in self.w.items()}}
+
     def parallelism(self):
         return (f"ep{self.world}: tokens data-parallel (8192 per rank), routed experts sharded, token all-to-all each way in forward and "
                 f"backward") if self.world > 1 else "single GPU (all 64 experts local)"
@@ -669,6 +688,21 @@ class Cfg5EpTrain:
 
 
 GPU_WORKLOADS = {"cfg2": Cfg2Prefill, "cfg3": Cfg3Decode, "cfg4": Cfg4LongPrefill, "cfg5": Cfg5EpTrain}
+
+
+def dump_outputs(outs, out_dir):
+    """float32 copies of the tensors in `outs` as out_dir/<name>.npy, within DUMP_BUDGET bytes in all: a tensor of more than
+    its share of the budget is written as a seeded sample of its elements (flattened; the same positions in every run)."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    cap = (DUMP_BUDGET // len(outs) - 1024) // 4       # 1 KB per file for the .npy header
+    for name, t in outs.items():
+        t = t.detach()
+        if t.numel() > cap:
+            idx = torch.randint(t.numel(), (cap,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 def run_aria(args, rank, local_rank, world):
@@ -696,14 +730,15 @@ def run_aria(args, rank, local_rank, world):
         torch.cuda.synchronize()
 
     def timed(fn, n):
+        """(ms per call, what the last call returned) over n calls"""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(n):
-            fn()
+            out = fn()
         e1.record()
         barrier()
-        return e0.elapsed_time(e1) / n
+        return e0.elapsed_time(e1) / n, out
 
     for _ in range(warmup):
         wl.step_resident()
@@ -713,19 +748,21 @@ def run_aria(args, rank, local_rank, world):
     l0 = L.launch_count
     wl.step_eager()       # kernels per step (counted on one eager step; the graph replays exactly these launches)
     launches_per_step = L.launch_count - l0
-    ms = timed(wl.step_resident, steps)
+    ms, out = timed(wl.step_resident, steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(wl.outputs(out), args.dump_outputs)
 
     # per-kernel table: CUDA events around every C-ABI call of K eager steps (events cannot be recorded inside a graph replay)
     kernels, ms_eager = None, None
     if not args.no_kernel_table:
         with KernelTable(torch, ops) as kt:
-            ms_eager = timed(wl.step_eager, steps)
+            ms_eager, _ = timed(wl.step_eager, steps)
         peaks, peak_src = _peaks()
         kernels = kt.table(steps, ms_eager, peaks)
 
     for _ in range(2):
         wl.step_e2e()
-    ms_e2e = timed(wl.step_e2e, steps)
+    ms_e2e, _ = timed(wl.step_e2e, steps)
     clocks = sampler.stop()
 
     if world > 1:
@@ -784,7 +821,13 @@ def main():
                     help="N > 1: shard the routed experts over the ranks (default for cfg2/cfg5) or run independent replicas")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-kernel-table", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "aria":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl aria)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

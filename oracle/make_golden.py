@@ -1,10 +1,10 @@
 """TEST INFRASTRUCTURE — generate tests/golden/*.pt by running the UNMODIFIED reference modules
-(loaded from /root/reference by oracle/ref_loader.py) on CPU with seeded random weights.
+(loaded by oracle/ref_loader.py; ARIA_REFERENCE_ROOT names a checkout of rhymes-ai/Aria) on CPU with seeded random weights.
 
-Run in the build container (the GPU box has no /root/reference):
-    python oracle/make_golden.py
+    ARIA_REFERENCE_ROOT=<Aria checkout> python oracle/make_golden.py
 Each fixture stores inputs, the reference outputs (and MoE intermediates), and the weight checksum;
-weights are re-created from the seed by oracle/configs.py.
+weights are re-created from the seed by oracle/configs.py.  Large gradients are stored as a strided sample (`flat[::stride]`,
+stride stored beside them; see strided_sample) so that the fixtures stay small.
 """
 import os
 import sys
@@ -17,6 +17,13 @@ from oracle import configs as C  # noqa: E402
 from oracle.ref_loader import load_reference  # noqa: E402
 
 OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
+GRAD_SAMPLE = 4096
+
+
+def strided_sample(t, n=GRAD_SAMPLE):
+    """(flat[::stride], stride) with stride the smallest that leaves at most n elements; tests compare the same positions."""
+    stride = -(-t.numel() // n)
+    return t.detach().reshape(-1)[::stride].clone(), stride
 
 
 def build_reference_model(ref, cfg, sd, dtype):
@@ -115,7 +122,7 @@ def main():
     for dtype, tag in ((torch.float32, "fp32"), (torch.bfloat16, "bf16")):
         gen = torch.Generator().manual_seed(3)
         ttc = dict(hidden_size=128, moe_num_experts=8, moe_topk=2, moe_intermediate_size=64, moe_num_shared_experts=2)
-        sd = C.moe_layer_state(ttc, gen)                    # small layer: the fixture stores every parameter gradient
+        sd = C.moe_layer_state(ttc, gen)                    # small layer: the fixture stores a sample of every parameter gradient
         sd["router.weight"] = sd["router.weight"] * 20      # spread the logits so the loss terms are well above rounding noise
         x = torch.randn(2, 16, 128, generator=gen)
         dout = torch.randn(2, 16, 128, generator=gen)
@@ -134,7 +141,7 @@ def main():
                 out.backward(dout)
             finally:
                 ref.moe_lm.MoEAuxLossAutoScaler.set_loss_scale(torch.tensor(1.0))
-            grads = {n: p.grad.detach().clone() for n, p in layer.named_parameters()}
+            grads = {n: strided_sample(p.grad) for n, p in layer.named_parameters()}
             w = {n: v.clone().requires_grad_(True) for n, v in sd.items()}
             xo = x.clone().requires_grad_(True)
             O._LossGradInjector.scale = scale
@@ -142,9 +149,10 @@ def main():
                 O.moe_layer(xo, w, 2, loss_coeffs=(z_c, aux_c)).backward(dout)
             finally:
                 O._LossGradInjector.scale = 1.0
-        err = max(float((grads[n].float() - w[n].grad.float()).abs().max()) for n in grads)
+        err = max(float((g.float() - w[n].grad.reshape(-1)[::st].float()).abs().max()) for n, (g, st) in grads.items())
         report.append(f"moe_layer train-mode grads {tag}: oracle-vs-reference max abs err over parameter grads {err:.3e}")
-        torch.save(dict(x=x, dout=dout, out=out.detach(), grads=grads, dx=xr.grad.detach(), z_coeff=z_c, aux_coeff=aux_c,
+        torch.save(dict(x=x, dout=dout, out=out.detach(), grads={n: g for n, (g, _) in grads.items()},
+                        grad_strides={n: st for n, (_, st) in grads.items()}, dx=xr.grad.detach(), z_coeff=z_c, aux_coeff=aux_c,
                         loss_scale=scale, checksum=C.state_checksum(sd), seed=3, text_config=ttc),
                    os.path.join(OUT, f"moe_layer_train_{tag}.pt"))
 
@@ -201,6 +209,83 @@ def main():
             torch.save(dict(input_ids=ids, pixel_values=pv, pixel_mask=pm, vit=vit_h, image_attn_mask=img_mask,
                             projector=proj, logits=logits, checksum=C.state_checksum(sd), seed=0),
                        os.path.join(OUT, f"aria_tiny_{tag}_{'masked' if masked else 'full'}.pt"))
+
+    # ---- (3) the cases of tests/test_oracle_vs_reference.py: same seeds and shapes as the tests, reference outputs only ----
+    live = {}
+    for dtype, tag in ((torch.float32, "fp32"), (torch.bfloat16, "bf16")):
+        for T, E, k in ((1, 8, 2), (7, 8, 2), (64, 16, 6), (33, 64, 6)):
+            tc = dict(hidden_size=128, moe_num_experts=E, moe_topk=k, moe_intermediate_size=64, moe_num_shared_experts=2)
+            gen = torch.Generator().manual_seed(T * 131 + E)
+            sd = {n: v.to(dtype) for n, v in C.moe_layer_state(tc, gen).items()}
+            x = torch.randn(1, T, 128, generator=gen).to(dtype)
+            layer = ref.moe_lm.MoELayer(ref.moe_lm.AriaMoELMConfig(**tc))
+            layer.load_state_dict(sd, strict=True)
+            layer = layer.to(dtype).eval()
+            _, ridx, _ = layer.router(x)
+            live[f"{tag}_T{T}_E{E}_k{k}"] = dict(out=layer(x), top_idx=ridx, checksum=C.state_checksum(sd),
+                                                 x_checksum=float(x.double().sum()))
+    torch.save(live, os.path.join(OUT, "moe_layer_live.pt"))
+
+    train_live = {}
+    for dtype, tag in ((torch.float32, "fp32"), (torch.bfloat16, "bf16")):
+        T, E, k, d = 48, 16, 4, 128
+        tc = dict(hidden_size=d, moe_num_experts=E, moe_topk=k, moe_intermediate_size=64, moe_num_shared_experts=2,
+                  moe_z_loss_coeff=0.5, moe_aux_loss_coeff=2.0)
+        gen = torch.Generator().manual_seed(5)
+        sd = {n: v.to(dtype) for n, v in C.moe_layer_state(tc, gen).items()}
+        sd["router.weight"] = (sd["router.weight"].float() * 20).to(dtype)
+        x0 = torch.randn(1, T, d, generator=gen).to(dtype)
+        dout = torch.randn(1, T, d, generator=gen).to(dtype)
+        fix = dict(checksum=C.state_checksum(sd), x_checksum=float(x0.double().sum()) + float(dout.double().sum()))
+        for scale in (1.0, 64.0):
+            with torch.enable_grad():
+                layer = ref.moe_lm.MoELayer(ref.moe_lm.AriaMoELMConfig(**tc))
+                layer.load_state_dict(sd, strict=True)
+                layer = layer.to(dtype).train()
+                ref.moe_lm.MoEAuxLossAutoScaler.set_loss_scale(torch.tensor(scale))
+                try:
+                    xr = x0.clone().requires_grad_(True)
+                    layer(xr).backward(dout)
+                finally:
+                    ref.moe_lm.MoEAuxLossAutoScaler.set_loss_scale(torch.tensor(1.0))
+            grads = {n: strided_sample(p.grad, 1024) for n, p in layer.named_parameters()}
+            fix[scale] = dict(grads={n: g for n, (g, _) in grads.items()}, grad_strides={n: st for n, (_, st) in grads.items()},
+                              grad_absmax={n: float(p.grad.float().abs().max()) for n, p in layer.named_parameters()},
+                              dx=xr.grad.detach())
+        train_live[tag] = fix
+    torch.save(train_live, os.path.join(OUT, "moe_layer_train_live.pt"))
+
+    lora_live = {}
+    for dtype, tag in ((torch.float32, "fp32"), (torch.bfloat16, "bf16")):
+        g = torch.Generator().manual_seed(4)
+        E, K, N, r, alpha = 4, 64, 96, 8, 32
+        counts = torch.tensor([16, 0, 40, 24])
+        rows = int(counts.sum())
+        w = (torch.randn(E, K, N, generator=g) * 0.05).to(dtype)
+        a = (torch.randn(E, K, r, generator=g) * 0.05).to(dtype)
+        b = (torch.randn(E, r, N, generator=g) * 0.05).to(dtype)
+        x0 = torch.randn(rows, K, generator=g).to(dtype)
+        dy = torch.randn(rows, N, generator=g).to(dtype)
+        with torch.enable_grad():
+            base = ref.moe_lm.GroupedGEMM(K, N, E)
+            layer = lora_mod.GroupedGemmLoraLayer(base, "default", r=r, lora_alpha=alpha).to(dtype)
+            with torch.no_grad():
+                base.weight.copy_(w)
+                layer.lora_A["default"].weight.copy_(a)
+                layer.lora_B["default"].weight.copy_(b)
+            xr = x0.clone().requires_grad_(True)
+            out = layer(xr, counts)
+            out.backward(dy)
+        fix = dict(x_checksum=float(x0.double().sum()), scaling=layer.scaling["default"], out=out.detach(),
+                   d_a=layer.lora_A["default"].weight.grad.detach(), d_b=layer.lora_B["default"].weight.grad.detach(),
+                   dx=xr.grad.detach())
+        if dtype == torch.float32:
+            with torch.no_grad():
+                layer.merge()
+                merged_weight, stride = strided_sample(base.weight)
+                fix.update(merged_out=layer(x0, counts), merged_weight=merged_weight, merged_weight_stride=stride)
+        lora_live[tag] = fix
+    torch.save(lora_live, os.path.join(OUT, "lora_layer_live.pt"))
     print("\n".join(report))
     with open(os.path.join(OUT, "REPORT.txt"), "w") as f:
         f.write("oracle/make_golden.py — oracle restatement vs unmodified reference, at generation time\n")

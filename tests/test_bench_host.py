@@ -103,3 +103,20 @@ def test_dominant_kernels_have_committed_dram_traffic():
     assert t_attn and t_fc1 and b._traffic_for("no_such_kernel[1]") is None
     assert 45158400 <= t_attn <= 1.6 * 45158400          # q, k, v, out of 16 heads x 4900 x 72 (+ stream-K pieces)
     assert 1129447424 * 0.98 <= t_fc1 <= 1.05 * 1129447424
+
+
+def test_dump_outputs_stays_within_budget_and_samples_the_same_positions(tmp_path):
+    import numpy as np
+    import torch
+    b = _bench()
+    b.DUMP_BUDGET = 1 << 16
+    big = torch.randn(100000, generator=torch.Generator().manual_seed(1))
+    outs = {"logits": torch.arange(6.0).reshape(2, 3).bfloat16(), "dx": big}
+    for run in ("a", "b"):
+        b.dump_outputs(outs, str(tmp_path / run))
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= b.DUMP_BUDGET
+    small = np.load(tmp_path / "a" / "logits.npy")
+    assert small.dtype == np.float32 and small.shape == (2, 3) and (small == np.arange(6.0).reshape(2, 3)).all()
+    sample_a, sample_b = np.load(tmp_path / "a" / "dx.npy"), np.load(tmp_path / "b" / "dx.npy")
+    assert sample_a.dtype == np.float32 and 0 < sample_a.size < big.numel()
+    assert (sample_a == sample_b).all() and np.isin(sample_a, big.numpy()).all()
