@@ -85,6 +85,13 @@ SIGNATURES = {
     "aria_attention_fwd_workspace_bytes": (i64, [i32, i32, i32, i32, i32, i32]),
     "aria_attention_decode": (i32, [vp, vp, vp, vp, vp, i32, i32, i32, i64, i64, i64, i64, f32, vp, i64, vp]),
     "aria_attention_decode_workspace_bytes": (i64, [i32, i32, i32]),
+    "aria_attention_fwd_lse": (i32, [vp, vp, vp, vp, vp, vp, i32, i32, i32, i64, i64, i64, i64, f32, i32, i32, vp]),
+    "aria_attention_bwd_workspace_bytes": (i64, [i32, i32, i32]),
+    "aria_attention_bwd": (i32, [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i64, i64, i64, i64, f32, i32, i32, vp, i64,
+                                 vp]),
+    "aria_rmsnorm_bwd_workspace_bytes": (i64, [i64, i32]),
+    "aria_rmsnorm_bwd": (i32, [vp, vp, vp, vp, vp, vp, i64, i32, f32, vp, i64, vp]),
+    "aria_rope_bwd": (i32, [vp, vp, vp, vp, i64, i32, i32, vp]),
 }
 
 _lib = None
@@ -109,7 +116,7 @@ def load():
 
 
 # kernels launched per C-ABI call (for bench.py's `gpu_launches`; memsets are not counted)
-KERNELS_PER_CALL = {"router_topk": 2, "attention_decode": 2, "moe_block_fwd": 9}
+KERNELS_PER_CALL = {"router_topk": 2, "attention_decode": 2, "moe_block_fwd": 9, "attention_bwd": 3, "rmsnorm_bwd": 2}
 # kernels exported for A/B measurements only (scripts/), not part of include/aria_b200.h
 EXTRA_SIGNATURES = {
     "aria_attention_fwd_v2": (i32, [vp, vp, vp, vp, vp, i32, i32, i32, i32, i64, i64, i64, i64, i32, f32, i32, vp]),

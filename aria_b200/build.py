@@ -10,7 +10,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libaria_b200.so")
-SOURCES = ["gemm.cu", "gemm2.cu", "gemm_wgrad.cu", "moe_route.cu", "moe_block.cu", "moe_bwd.cu", "ep.cu", "elementwise.cu", "attention.cu", "attention_v3.cu"]
+SOURCES = ["gemm.cu", "gemm2.cu", "gemm_wgrad.cu", "moe_route.cu", "moe_block.cu", "moe_bwd.cu", "ep.cu", "elementwise.cu", "attention.cu", "attention_v3.cu", "attention_bwd.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr", "-Xptxas", "-v",

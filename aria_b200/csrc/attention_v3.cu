@@ -68,6 +68,7 @@ struct Attn3Params {
   const uint8_t* key_mask;  // [B, Tk] 1 = masked out
   __nv_bfloat16* out;       // [B, Tq, H*out_hd]
   float* partial;           // [slots][256][HD + 4] fp32 (O unnormalised | m | l | pad), stream-K pieces
+  float* lse;               // [B, H, Tq] fp32 (LSE instantiations only): m + log2(l), +INF for a row without a visible key
   int n_q_pairs, n_kv_all;
   int units, n_cta, full_rounds, leftover, split;  // work distribution (see header)
 };
@@ -116,7 +117,9 @@ ARIA_DEVICE bool get_item(const Attn3Params& p, int c, int i, WorkItem& w) {
   return true;
 }
 
-template <int HD, int W, bool CAUSAL>
+// LSE: the epilogue also stores each row's softmax normaliser in the log2 domain of scale*log2e*s the kernel tracks
+// (the attention backward's input); whole units only (no stream-K pieces).
+template <int HD, int W, bool CAUSAL, bool LSE = false>
 __global__ void __launch_bounds__(A3_THREADS, 1)
 attn_fwd3_kernel(const __grid_constant__ CUtensorMap tmQ0, const __grid_constant__ CUtensorMap tmQ1,
                  const __grid_constant__ CUtensorMap tmK0, const __grid_constant__ CUtensorMap tmK1,
@@ -496,6 +499,7 @@ attn_fwd3_kernel(const __grid_constant__ CUtensorMap tmQ0, const __grid_constant
       tc_fence_after();
       if (w.slot < 0) {
         const float inv_l = l > 0.f ? 1.0f / l : 0.f;
+        if (LSE && row_ok) p.lse[static_cast<int64_t>(w.bh) * p.Tq + q] = l > 0.f ? m_ref + log2f(l) : INFINITY;
         __nv_bfloat16* orow = p.out + (static_cast<int64_t>(b) * p.Tq + q) * (static_cast<int64_t>(p.H) * p.out_hd) + h * p.out_hd;
 #pragma unroll 1
         for (int c = 0; c < HD; c += 16) {
@@ -601,7 +605,7 @@ static int make_tmap_heads3(CUtensorMap* tm, const void* ptr, int T, int H, int 
   return make_tmap_bf16_swz(tm, ptr, 4, dims, str, box, swz);
 }
 
-template <int HD, int W, bool CAUSAL>
+template <int HD, int W, bool CAUSAL, bool LSE = false>
 static int launch_attn3(const void* q, const void* k, const void* v, Attn3Params& p, int64_t q_stride_b, int64_t q_stride_h,
                         int64_t kv_stride_b, int64_t kv_stride_h, cudaStream_t stream) {
   using C = A3Cfg<HD, W>;
@@ -622,7 +626,7 @@ static int launch_attn3(const void* q, const void* k, const void* v, Attn3Params
     rc = make_tmap_heads3(&tmV, v, p.Tk, p.H, p.B, kv_stride_b, kv_stride_h, 64, CU_TENSOR_MAP_SWIZZLE_128B);
   }
   if (rc) return rc;
-  auto kern = attn_fwd3_kernel<HD, W, CAUSAL>;
+  auto kern = attn_fwd3_kernel<HD, W, CAUSAL, LSE>;
   static bool attr_set[kMaxDevices] = {};
   if (ensure_dynamic_smem(attr_set, kern, C::SMEM) != cudaSuccess) return ARIA_ERR_CUDA;
   kern<<<p.n_cta, A3_THREADS, C::SMEM, stream>>>(tmQ0, tmQ1, tmK0, tmK1, tmV, p);
@@ -717,4 +721,39 @@ extern "C" int aria_attention_fwd(const void* q, const void* k, const void* v, v
   if (hd == 80) ARIA_A3(80, 128);
   ARIA_A3(128, 128);
 #undef ARIA_A3
+}
+
+// Causal self-attention forward that also returns lse (aria_attention_bwd's input): the v3 kernel with one unit per CTA,
+// heaviest first, exactly as aria_attention_fwd runs causal launches that it does not route to the round-1 kernel.
+extern "C" int aria_attention_fwd_lse(const void* q, const void* k, const void* v, void* out, float* lse, const uint8_t* key_mask,
+                                      int32_t B, int32_t H, int32_t T, int64_t q_stride_b, int64_t q_stride_h, int64_t kv_stride_b,
+                                      int64_t kv_stride_h, float scale, int32_t head_dim, int32_t causal, aria_stream_t stream_) {
+  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+  if (!causal || head_dim != 128) {
+    fprintf(stderr, "aria_b200: attention forward with lse supports causal self-attention with head_dim 128 only\n");
+    return ARIA_ERR_UNSUPPORTED;
+  }
+  ARIA_CHECK_ARG(q && k && v && out && lse);
+  ARIA_CHECK_ARG(B > 0 && H > 0 && T > 0);
+  ARIA_CHECK_ARG(q_stride_b % 8 == 0 && q_stride_h % 8 == 0 && kv_stride_b % 8 == 0 && kv_stride_h % 8 == 0);
+  Attn3Params p{};
+  p.B = B;
+  p.H = H;
+  p.Tq = T;
+  p.Tk = T;
+  p.out_hd = 128;
+  p.scale_log2 = scale * 1.4426950408889634f;
+  p.key_mask = key_mask;
+  p.out = static_cast<__nv_bfloat16*>(out);
+  p.lse = lse;
+  p.n_q_pairs = (T + 2 * A3_BM - 1) / (2 * A3_BM);
+  p.n_kv_all = (T + A3_BN - 1) / A3_BN;
+  const int64_t units = static_cast<int64_t>(B) * H * p.n_q_pairs;
+  ARIA_CHECK_ARG(units < (1ll << 31));
+  p.units = static_cast<int>(units);
+  p.n_cta = p.units;
+  p.full_rounds = 1;
+  p.leftover = 0;
+  p.split = 1;
+  return launch_attn3<128, 128, true, true>(q, k, v, p, q_stride_b, q_stride_h, kv_stride_b, kv_stride_h, stream);
 }

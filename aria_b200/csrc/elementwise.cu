@@ -322,6 +322,134 @@ __global__ void __launch_bounds__(256) add_pos_kernel(const uint4* __restrict__ 
   }
 }
 
+
+// Backward of rmsnorm_kernel without residual (LlamaRMSNorm autograd): y = w o bf16(x r), r = rsqrt(mean(x^2) + eps).
+//   dx = r (g - x r^2 mean(g o x)) (+ dres),  g = dy o w;   dw = sum_rows dy o bf16(x r)
+// One 128-thread block per row (grid-stride over rows); dw is accumulated per block in registers and written as fp32 partials
+// [gridDim.x][d] that rmsnorm_dw_reduce_kernel sums in a fixed order: deterministic, no atomics.
+constexpr int RMS_BWD_BLOCKS = 256;  // fixed, so that the workspace size does not depend on the device
+template <int MAXV>
+__global__ void __launch_bounds__(128) rmsnorm_bwd_kernel(const uint4* __restrict__ x, const uint4* __restrict__ w,
+                                                          const uint4* __restrict__ dy, const uint4* __restrict__ dres,
+                                                          uint4* __restrict__ dx, float* __restrict__ partial, int64_t rows, int vpr,
+                                                          float eps, float inv_d) {
+  __shared__ float red[2][4];
+  const int tid = threadIdx.x;
+  float dw[MAXV][8];
+#pragma unroll
+  for (int i = 0; i < MAXV; ++i)
+#pragma unroll
+    for (int j = 0; j < 8; ++j) dw[i][j] = 0.f;
+  for (int64_t r = blockIdx.x; r < rows; r += gridDim.x) {
+    float h[MAXV][8], g[MAXV][8];
+    float ss = 0.f, sg = 0.f;
+#pragma unroll
+    for (int i = 0; i < MAXV; ++i) {
+      const int v = tid + i * 128;
+      if (v < vpr) {
+        const uint4 qx = x[r * vpr + v], qy = dy[r * vpr + v], qw = __ldg(w + v);
+        const uint32_t a[4] = {qx.x, qx.y, qx.z, qx.w}, b[4] = {qy.x, qy.y, qy.z, qy.w}, c[4] = {qw.x, qw.y, qw.z, qw.w};
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          h[i][2 * j] = bf16_lo(a[j]);
+          h[i][2 * j + 1] = bf16_hi(a[j]);
+          g[i][2 * j] = bf16_lo(b[j]);       // dy for now; g = dy o w below
+          g[i][2 * j + 1] = bf16_hi(b[j]);
+          const float w0 = bf16_lo(c[j]), w1 = bf16_hi(c[j]);
+          ss += h[i][2 * j] * h[i][2 * j] + h[i][2 * j + 1] * h[i][2 * j + 1];
+          sg += g[i][2 * j] * w0 * h[i][2 * j] + g[i][2 * j + 1] * w1 * h[i][2 * j + 1];
+        }
+      }
+    }
+    ss = warp_sum(ss);
+    sg = warp_sum(sg);
+    __syncthreads();  // red[] free (previous row consumed)
+    if ((tid & 31) == 0) {
+      red[0][tid >> 5] = ss;
+      red[1][tid >> 5] = sg;
+    }
+    __syncthreads();
+    ss = red[0][0] + red[0][1] + red[0][2] + red[0][3];
+    sg = red[1][0] + red[1][1] + red[1][2] + red[1][3];
+    const float rstd = 1.0f / sqrtf(ss * inv_d + eps);   // as the forward computes it
+    const float c2 = rstd * rstd * sg * inv_d;
+#pragma unroll
+    for (int i = 0; i < MAXV; ++i) {
+      const int v = tid + i * 128;
+      if (v < vpr) {
+        const uint4 qw = __ldg(w + v);
+        const uint32_t c[4] = {qw.x, qw.y, qw.z, qw.w};
+        float res[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+        if (dres) {
+          const uint4 qr = dres[r * vpr + v];
+          const uint32_t e[4] = {qr.x, qr.y, qr.z, qr.w};
+#pragma unroll
+          for (int j = 0; j < 4; ++j) {
+            res[2 * j] = bf16_lo(e[j]);
+            res[2 * j + 1] = bf16_hi(e[j]);
+          }
+        }
+        float o[8];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          const float wj = (j & 1) ? bf16_hi(c[j >> 1]) : bf16_lo(c[j >> 1]);
+          dw[i][j] += g[i][j] * bf16r(h[i][j] * rstd);
+          o[j] = rstd * (g[i][j] * wj - h[i][j] * c2) + res[j];
+        }
+        dx[r * vpr + v] = make_uint4(pack_bf16(o[0], o[1]), pack_bf16(o[2], o[3]), pack_bf16(o[4], o[5]), pack_bf16(o[6], o[7]));
+      }
+    }
+  }
+#pragma unroll
+  for (int i = 0; i < MAXV; ++i) {
+    const int v = tid + i * 128;
+    if (v < vpr) {
+      float4* dst = reinterpret_cast<float4*>(partial + static_cast<int64_t>(blockIdx.x) * vpr * 8 + v * 8);
+      dst[0] = make_float4(dw[i][0], dw[i][1], dw[i][2], dw[i][3]);
+      dst[1] = make_float4(dw[i][4], dw[i][5], dw[i][6], dw[i][7]);
+    }
+  }
+}
+
+// dw[c] = bf16(sum_b partial[b][c]), blocks summed in index order
+__global__ void __launch_bounds__(256) rmsnorm_dw_reduce_kernel(const float* __restrict__ partial, __nv_bfloat16* __restrict__ dw,
+                                                                int n_part, int d) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= d) return;
+  float s = 0.f;
+  for (int b = 0; b < n_part; ++b) s += partial[static_cast<int64_t>(b) * d + c];
+  dw[c] = __float2bfloat16_rn(s);
+}
+
+// Transpose of rotate-half RoPE, in place on token-major [rows, n_heads*128]: dx1 = dy1 c + dy2 s, dx2 = dy2 c - dy1 s.
+// One warp per (row, head); lane l owns dims 2l, 2l+1 of each half.
+__global__ void __launch_bounds__(256) rope_bwd_kernel(uint32_t* __restrict__ x, const uint32_t* __restrict__ cos_t,
+                                                       const uint32_t* __restrict__ sin_t, const int32_t* __restrict__ position_ids,
+                                                       int64_t rows, int n_heads, int rows_per_batch) {
+  const int lane = threadIdx.x & 31;
+  const int64_t wid = static_cast<int64_t>(blockIdx.x) * 8 + (threadIdx.x >> 5);
+  if (wid >= rows * n_heads) return;
+  const int64_t r = wid / n_heads;
+  const int pos = position_ids ? position_ids[r] : static_cast<int>(r % rows_per_batch);
+  uint32_t* row = x + wid * 64;                    // 128 bf16 = 64 words
+  const uint32_t* cs = cos_t + static_cast<int64_t>(pos) * 64;
+  const uint32_t* sn = sin_t + static_cast<int64_t>(pos) * 64;
+  const uint32_t a = row[lane], b = row[32 + lane];
+  const uint32_t c1 = __ldg(cs + lane), c2 = __ldg(cs + 32 + lane), s1 = __ldg(sn + lane), s2 = __ldg(sn + 32 + lane);
+  const float y1[2] = {bf16_lo(a), bf16_hi(a)}, y2[2] = {bf16_lo(b), bf16_hi(b)};
+  const float co1[2] = {bf16_lo(c1), bf16_hi(c1)}, co2[2] = {bf16_lo(c2), bf16_hi(c2)};
+  const float si1[2] = {bf16_lo(s1), bf16_hi(s1)}, si2[2] = {bf16_lo(s2), bf16_hi(s2)};
+  float o1[2], o2[2];
+#pragma unroll
+  for (int u = 0; u < 2; ++u) {
+    // forward: out1 = x1 c1 - x2 s1, out2 = x2 c2 + x1 s2
+    o1[u] = y1[u] * co1[u] + y2[u] * si2[u];
+    o2[u] = y2[u] * co2[u] - y1[u] * si1[u];
+  }
+  row[lane] = pack_bf16(o1[0], o1[1]);
+  row[32 + lane] = pack_bf16(o2[0], o2[1]);
+}
+
 }  // namespace aria
 
 using namespace aria;
@@ -485,4 +613,45 @@ extern "C" int aria_ipc_open(const void* handle64, void** base_out) {
 
 extern "C" int aria_ipc_close(void* base) {
   return cudaIpcCloseMemHandle(base) == cudaSuccess ? ARIA_OK : ARIA_ERR_CUDA;
+}
+
+extern "C" int64_t aria_rmsnorm_bwd_workspace_bytes(int64_t rows, int32_t d) {
+  if (rows <= 0 || d <= 0 || d % 8) return ARIA_ERR_BAD_ARG;
+  const int64_t blocks = rows < RMS_BWD_BLOCKS ? rows : RMS_BWD_BLOCKS;
+  return blocks * d * static_cast<int64_t>(sizeof(float));
+}
+
+extern "C" int aria_rmsnorm_bwd(const void* x, const void* weight, const void* dy, const void* dres, void* dx, void* dw, int64_t rows,
+                                int32_t d, float eps, void* workspace, int64_t workspace_bytes, aria_stream_t stream_) {
+  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+  ARIA_CHECK_ARG(x && weight && dy && dx && dw && workspace && d > 0 && d % 8 == 0 && d <= 128 * 8 * 4 && rows > 0);
+  ARIA_CHECK_ARG(workspace_bytes >= aria_rmsnorm_bwd_workspace_bytes(rows, d));
+  const int vpr = d / 8;
+  const int grid = static_cast<int>(rows < RMS_BWD_BLOCKS ? rows : RMS_BWD_BLOCKS);
+  float* partial = static_cast<float*>(workspace);
+#define RMSB(MAXV)                                                                                                          \
+  rmsnorm_bwd_kernel<MAXV><<<grid, 128, 0, stream>>>(static_cast<const uint4*>(x), static_cast<const uint4*>(weight),       \
+                                                     static_cast<const uint4*>(dy), static_cast<const uint4*>(dres),        \
+                                                     static_cast<uint4*>(dx), partial, rows, vpr, eps, 1.0f / d)
+  if (vpr <= 128) RMSB(1);
+  else if (vpr <= 256) RMSB(2);
+  else if (vpr <= 384) RMSB(3);
+  else RMSB(4);
+#undef RMSB
+  int rc = check_launch("rmsnorm_bwd_kernel");
+  if (rc) return rc;
+  rmsnorm_dw_reduce_kernel<<<(d + 255) / 256, 256, 0, stream>>>(partial, static_cast<__nv_bfloat16*>(dw), grid, d);
+  return check_launch("rmsnorm_dw_reduce_kernel");
+}
+
+extern "C" int aria_rope_bwd(void* x, const void* cos_t, const void* sin_t, const int32_t* position_ids, int64_t rows,
+                             int32_t n_heads, int32_t rows_per_batch, aria_stream_t stream_) {
+  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+  ARIA_CHECK_ARG(x && cos_t && sin_t && rows >= 0 && n_heads > 0 && (position_ids || rows_per_batch > 0));
+  if (rows == 0) return ARIA_OK;
+  const int64_t warps = rows * n_heads;
+  rope_bwd_kernel<<<static_cast<unsigned>((warps + 7) / 8), 256, 0, stream>>>(
+      static_cast<uint32_t*>(x), static_cast<const uint32_t*>(cos_t), static_cast<const uint32_t*>(sin_t), position_ids, rows, n_heads,
+      rows_per_batch);
+  return check_launch("rope_bwd_kernel");
 }

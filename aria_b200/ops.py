@@ -479,6 +479,42 @@ def rmsnorm(x: torch.Tensor, weight: torch.Tensor, eps: float, residual: Optiona
     return out if residual is None else (out, s)
 
 
+def rmsnorm_bwd(x: torch.Tensor, weight: torch.Tensor, dy: torch.Tensor, eps: float, dres: Optional[torch.Tensor] = None):
+    """Backward of rmsnorm(x, weight, eps) (no residual): -> (dx (+ dres), dw [d] bf16, deterministic reduction)."""
+    _chk(x), _chk(weight), _chk(dy)
+    d = x.shape[-1]
+    rows = x.numel() // d
+    assert dy.shape == x.shape and weight.numel() == d
+    if dres is not None:
+        _chk(dres)
+        assert dres.shape == x.shape
+    dx = torch.empty_like(x)
+    dw = torch.empty_like(weight)
+    lib = L.load()
+    nbytes = lib.aria_rmsnorm_bwd_workspace_bytes(rows, d)
+    ws = torch.empty((max(nbytes, 16),), dtype=torch.uint8, device=x.device)
+    with torch.cuda.device(x.device):
+        L.check(lib.aria_rmsnorm_bwd(_p(x), _p(weight), _p(dy), _p(dres), _p(dx), _p(dw), rows, d, eps, _p(ws), ws.numel(),
+                                     _stream(x)), "rmsnorm_bwd")
+    return dx, dw
+
+
+def rope_bwd(x: torch.Tensor, cos: torch.Tensor, sin: torch.Tensor, rows_per_batch: int,
+             position_ids: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """In place on token-major x [..., n_heads*128]: the transpose of rotate-half RoPE (gradient of the rotated q or k).
+    Positions: position_ids [rows] int32 when given, else row % rows_per_batch (the HEADS epilogue's convention)."""
+    _chk(x), _chk(cos), _chk(sin)
+    rows = x.numel() // x.shape[-1]
+    assert x.shape[-1] % 128 == 0 and cos.shape[-1] == 128
+    if position_ids is not None:
+        _chk(position_ids, torch.int32, align=4)
+        assert position_ids.numel() == rows
+    with torch.cuda.device(x.device):
+        L.check(L.load().aria_rope_bwd(_p(x), _p(cos), _p(sin), _p(position_ids), rows, x.shape[-1] // 128, rows_per_batch,
+                                       _stream(x)), "rope_bwd")
+    return x
+
+
 def layernorm(x: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor, eps: float) -> torch.Tensor:
     _chk(x), _chk(weight), _chk(bias)
     d = x.shape[-1]
@@ -563,6 +599,54 @@ def attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, Tq: int, Tk: in
                                        k.stride(0), k.stride(1), out_hd, scale, int(causal), _p(ws), ws_bytes, _stream(q)),
                 "attention_fwd")
     return out
+
+
+def _check_heads(*ts):
+    for t in ts:
+        if not (t.is_cuda and t.dtype == bf16 and t.dim() == 4 and t.stride(-1) == 1 and t.stride(-2) == 128 and t.shape[-1] == 128
+                and t.data_ptr() % 16 == 0):
+            raise RuntimeError("attention: q/k/v must be CUDA bf16 [B,H,T,128] with 128-element token rows (16-byte aligned)")
+
+
+def attention_fwd_lse(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, scale: float,
+                      key_mask: Optional[torch.Tensor] = None):
+    """Causal self-attention over q/k/v [B,H,T,128] -> (out [B,T,H*128] bf16, lse [B,H,T] fp32 in the log2 domain of
+    scale*log2(e)*s, +inf for a row that sees no key).  out equals `attention(..., causal=True)` where that takes the same kernel."""
+    _check_heads(q, k, v)
+    B, H, T = q.shape[0], q.shape[1], q.shape[2]
+    assert k.shape[:3] == (B, H, T) and k.stride() == v.stride()
+    out = torch.empty((B, T, H * 128), dtype=bf16, device=q.device)
+    lse = torch.empty((B, H, T), dtype=torch.float32, device=q.device)
+    if key_mask is not None:
+        _chk(key_mask, torch.uint8)
+        assert key_mask.shape == (B, T)
+    with torch.cuda.device(q.device):
+        L.check(L.load().aria_attention_fwd_lse(_p(q), _p(k), _p(v), _p(out), _p(lse), _p(key_mask), B, H, T, q.stride(0), q.stride(1),
+                                                k.stride(0), k.stride(1), scale, 128, 1, _stream(q)), "attention_fwd_lse")
+    return out, lse
+
+
+def attention_bwd(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, out: torch.Tensor, dout: torch.Tensor, lse: torch.Tensor,
+                  scale: float, key_mask: Optional[torch.Tensor] = None):
+    """Gradient of causal `attention_fwd_lse`: q/k/v [B,H,T,128] head-major, out / dout [B,T,H*128] token-major, lse [B,H,T]
+    -> (dq, dk, dv), each [B,T,H*128] token-major bf16 (gradients w.r.t. the q/k/v the attention consumed)."""
+    _check_heads(q, k, v)
+    B, H, T = q.shape[0], q.shape[1], q.shape[2]
+    assert k.shape[:3] == (B, H, T) and k.stride() == v.stride()
+    _chk(out), _chk(dout), _chk(lse, torch.float32)
+    assert out.shape == (B, T, H * 128) and dout.shape == out.shape and lse.shape == (B, H, T)
+    if key_mask is not None:
+        _chk(key_mask, torch.uint8)
+        assert key_mask.shape == (B, T)
+    dq, dk, dv = (torch.empty_like(out) for _ in range(3))
+    lib = L.load()
+    nbytes = lib.aria_attention_bwd_workspace_bytes(B, H, T)
+    ws = torch.empty((nbytes,), dtype=torch.uint8, device=q.device)
+    with torch.cuda.device(q.device):
+        L.check(lib.aria_attention_bwd(_p(q), _p(k), _p(v), _p(out), _p(dout), _p(lse), _p(dq), _p(dk), _p(dv), _p(key_mask), B, H, T,
+                                       q.stride(0), q.stride(1), k.stride(0), k.stride(1), scale, 128, 1, _p(ws), nbytes, _stream(q)),
+                "attention_bwd")
+    return dq, dk, dv
 
 
 def attention_v2(q, k, v, Tq, Tk, scale, causal, out_hd=128, key_mask=None):

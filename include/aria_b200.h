@@ -198,6 +198,20 @@ int aria_router_aux_bwd(const void* logits, const int32_t* counts, void* dlogits
  * If residual != NULL: first h = bf16(x + residual), written to sum_out, and the norm is taken of h. */
 int aria_rmsnorm(const void* x, const void* residual, const void* weight, void* out, void* sum_out, int64_t rows,
                  int32_t d, float eps, aria_stream_t stream);
+/* Backward of aria_rmsnorm without residual — replaces the autograd of LlamaRMSNorm (moe_lm.py:599-602):
+ *   dx = r * (g - x * r^2 * mean(g * x)) (+ dres),  g = dy * w,  r = rsqrt(mean(x^2) + eps);   dw = sum_rows dy * bf16(x * r).
+ * dres [rows, d] or NULL: the residual-stream gradient, added into dx in the same pass.  dw [d] bf16 is reduced
+ * deterministically through fp32 per-block partials in the workspace (no atomics).
+ * workspace: aria_rmsnorm_bwd_workspace_bytes(rows, d) = min(rows, 256) * d * 4 bytes. */
+int64_t aria_rmsnorm_bwd_workspace_bytes(int64_t rows, int32_t d);
+int aria_rmsnorm_bwd(const void* x, const void* weight, const void* dy, const void* dres, void* dx, void* dw, int64_t rows,
+                     int32_t d, float eps, void* workspace, int64_t workspace_bytes, aria_stream_t stream);
+/* Backward of rotate-half RoPE — replaces the autograd of apply_rotary_pos_emb (transformers modeling_llama), in place on
+ * token-major x [rows, n_heads*128] bf16: dx1 = dy1*cos + dy2*sin, dx2 = dy2*cos - dy1*sin (x1 / x2 = the two 64-wide halves
+ * of a head).  Positions as in the HEADS epilogue: position_ids[r] (int32) when given, else r % rows_per_batch; cos/sin
+ * tables from aria_rope_table. */
+int aria_rope_bwd(void* x, const void* cos, const void* sin, const int32_t* position_ids, int64_t rows, int32_t n_heads,
+                  int32_t rows_per_batch, aria_stream_t stream);
 /* nn.LayerNorm (Idefics2 encoder layers, projector): out = bf16((x-mean)*rstd*w + b). */
 int aria_layernorm(const void* x, const void* weight, const void* bias, void* out, int64_t rows, int32_t d,
                    float eps, aria_stream_t stream);
@@ -271,6 +285,25 @@ int aria_attention_decode(const void* q, const void* k, const void* v, void* out
                           int64_t q_stride_b, int64_t q_stride_h, int64_t kv_stride_b, int64_t kv_stride_h, float scale,
                           void* workspace, int64_t workspace_bytes, aria_stream_t stream);
 int64_t aria_attention_decode_workspace_bytes(int32_t B, int32_t H, int32_t Tk);
+/* Causal self-attention forward (Tq = Tk = T, head_dim 128) that also stores each query row's softmax normaliser — the
+ * forward half of the autograd of eager_attention_forward / SDPA behind moe_lm.py:594.  Layouts as aria_attention_fwd:
+ * q/k/v [B,H,T,128] head-major, out [B,T,H*128] token-major;  lse [B,H,T] fp32 = log2(sum_k 2^(s_k * scale * log2 e)) (the
+ * log2 domain of the scaled scores), +INF for a query row that sees no key.  out is bit-identical to aria_attention_fwd's
+ * for the launches that function runs on the same kernel (causal, T > 1024).  causal = 0 or head_dim != 128:
+ * ARIA_ERR_UNSUPPORTED. */
+int aria_attention_fwd_lse(const void* q, const void* k, const void* v, void* out, float* lse, const uint8_t* key_mask, int32_t B,
+                           int32_t H, int32_t T, int64_t q_stride_b, int64_t q_stride_h, int64_t kv_stride_b, int64_t kv_stride_h,
+                           float scale, int32_t head_dim, int32_t causal, aria_stream_t stream);
+/* Causal attention backward — replaces the autograd of eager_attention_forward / SDPA behind moe_lm.py:594.
+ *   q/k/v [B,H,T,128] head-major (the forward's buffers); out, dout, dq, dk, dv [B,T,H*128] token-major bf16 (the layout the
+ *   q/k/v projection GEMMs read back); lse from aria_attention_fwd_lse; key_mask [B,T] uint8 or NULL, 1 = masked out.
+ * Deterministic: repeated calls give bit-identical dq/dk/dv (no atomics).  causal = 0 or head_dim != 128:
+ * ARIA_ERR_UNSUPPORTED.  workspace: aria_attention_bwd_workspace_bytes(B, H, T) = Delta [B,H,T] fp32, rounded up to 256 B. */
+int64_t aria_attention_bwd_workspace_bytes(int32_t B, int32_t H, int32_t T);
+int aria_attention_bwd(const void* q, const void* k, const void* v, const void* out, const void* dout, const float* lse, void* dq,
+                       void* dk, void* dv, const uint8_t* key_mask, int32_t B, int32_t H, int32_t T, int64_t q_stride_b,
+                       int64_t q_stride_h, int64_t kv_stride_b, int64_t kv_stride_h, float scale, int32_t head_dim, int32_t causal,
+                       void* workspace, int64_t workspace_bytes, aria_stream_t stream);
 
 #ifdef __cplusplus
 }
