@@ -92,6 +92,12 @@ SIGNATURES = {
     "aria_rmsnorm_bwd_workspace_bytes": (i64, [i64, i32]),
     "aria_rmsnorm_bwd": (i32, [vp, vp, vp, vp, vp, vp, i64, i32, f32, vp, i64, vp]),
     "aria_rope_bwd": (i32, [vp, vp, vp, vp, i64, i32, i32, vp]),
+    "aria_lm_xent_fwd_workspace_bytes": (i64, [i64, i64]),
+    "aria_lm_xent_fwd": (i32, [vp, vp, vp, vp, vp, vp, i64, i64, i32, vp, i64, vp]),
+    "aria_lm_xent_bwd_workspace_bytes": (i64, [i64, i64, i32]),
+    "aria_lm_xent_bwd": (i32, [vp, vp, vp, vp, vp, vp, vp, vp, i64, i64, i32, vp, i64, vp]),
+    "aria_embedding_bwd_workspace_bytes": (i64, [i64, i64]),
+    "aria_embedding_bwd": (i32, [vp, vp, vp, i64, i32, i64, i64, vp, i64, vp]),
 }
 
 _lib = None
@@ -116,7 +122,8 @@ def load():
 
 
 # kernels launched per C-ABI call (for bench.py's `gpu_launches`; memsets are not counted)
-KERNELS_PER_CALL = {"router_topk": 2, "attention_decode": 2, "moe_block_fwd": 9, "attention_bwd": 3, "rmsnorm_bwd": 2}
+KERNELS_PER_CALL = {"router_topk": 2, "attention_decode": 2, "moe_block_fwd": 9, "attention_bwd": 3, "rmsnorm_bwd": 2,
+                    "lm_xent_fwd": 3, "embedding_bwd": 4}
 # kernels exported for A/B measurements only (scripts/), not part of include/aria_b200.h
 EXTRA_SIGNATURES = {
     "aria_attention_fwd_v2": (i32, [vp, vp, vp, vp, vp, i32, i32, i32, i32, i64, i64, i64, i64, i32, f32, i32, vp]),

@@ -235,9 +235,13 @@ int launch_gemm2_dispatch(int bn, bool b_mn, int epi, const CUtensorMap& tmA, co
 
 using namespace aria;
 
-extern "C" int aria_gemm(const aria_gemm_desc_t* d, aria_stream_t stream_) {
-  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+namespace aria {
+// aria_gemm with the epilogue given separately: `epi` may also be one of the internal modes of gemm_common.cuh (lm_loss.cu),
+// whose arguments come in `xp`.  Those run dense, single-segment GEMMs on 128-row A stages.
+int gemm_run(const aria_gemm_desc_t* d, int epi, const XentParams* xp, cudaStream_t stream) {
   ARIA_CHECK_ARG(d != nullptr);
+  const bool xent = epi >= EPI_XENT_STATS;
+  if (xent) ARIA_CHECK_ARG(xp != nullptr && d->n_seg == 1 && d->num_groups == 1 && d->residual == nullptr);
   ARIA_CHECK_ARG(d->a && d->b[0] && d->out[0]);
   ARIA_CHECK_ARG(d->m >= 0 && d->n > 0 && d->k > 0);
   ARIA_CHECK_ARG(d->n % 8 == 0 && d->k % 8 == 0 && d->lda % 8 == 0);
@@ -247,22 +251,23 @@ extern "C" int aria_gemm(const aria_gemm_desc_t* d, aria_stream_t stream_) {
   if (d->m == 0) return ARIA_OK;
   const bool b_mn = d->b_layout == ARIA_B_GKN;
   const bool b_gnk = d->b_layout == ARIA_B_GNK;
-  const bool swiglu = d->epilogue == ARIA_EPI_SWIGLU;
+  const bool swiglu = epi == ARIA_EPI_SWIGLU;
   if (b_mn) {
     ARIA_CHECK_ARG(d->n_seg == 1);
     // k-blocks must not straddle experts in the flattened [G*K, N] view (a single group has no neighbour: TMA zero-fills)
     ARIA_CHECK_ARG(d->k % BK == 0 || (d->num_groups == 1 && d->group_mod == 0));
     ARIA_CHECK_ARG(d->n % 64 == 0);
-    ARIA_CHECK_ARG(d->epilogue != ARIA_EPI_HEADS);
+    ARIA_CHECK_ARG(epi != ARIA_EPI_HEADS);
   } else {
     ARIA_CHECK_ARG(d->num_groups == 1 || d->n_seg == 1);
     if (swiglu) ARIA_CHECK_ARG(d->n_seg == 2 && d->b[1]);
-    if (b_gnk) ARIA_CHECK_ARG(d->n_seg == 1 && !swiglu && d->epilogue == ARIA_EPI_LINEAR && d->n % 128 == 0);
+    if (b_gnk) ARIA_CHECK_ARG(d->n_seg == 1 && !swiglu && epi == ARIA_EPI_LINEAR && d->n % 128 == 0);
     else ARIA_CHECK_ARG(d->num_groups == 1);
   }
   if (d->num_groups > 1) ARIA_CHECK_ARG(d->group_offsets != nullptr);
   if (d->group_counts) ARIA_CHECK_ARG(d->group_offsets != nullptr);
-  if (d->out_group_base) ARIA_CHECK_ARG(d->out_group_row0 != nullptr && d->epilogue == ARIA_EPI_LINEAR && d->group_offsets != nullptr);
+  if (xent) ARIA_CHECK_ARG(epi == EPI_ACC_F32 ? b_mn : !b_mn && !b_gnk);
+  if (d->out_group_base) ARIA_CHECK_ARG(d->out_group_row0 != nullptr && epi == ARIA_EPI_LINEAR && d->group_offsets != nullptr);
   ARIA_CHECK_ARG(d->a_rows == 0 || d->a_rows >= d->m);
 
   GemmParams p{};
@@ -299,6 +304,7 @@ extern "C" int aria_gemm(const aria_gemm_desc_t* d, aria_stream_t stream_) {
   p.dbg_lbo = d->dbg_lbo;
   p.dbg_sbo = d->dbg_sbo;
   p.dbg_kadv = d->dbg_kadv;
+  if (xent) p.x = *xp;
 
   // ---- kernel / tile shape selection
   // 2-CTA pairs (M=256 tiles, gemm2.cu) whenever there are at least two 128-row tiles of work per group; the 1-CTA
@@ -315,7 +321,7 @@ extern "C" int aria_gemm(const aria_gemm_desc_t* d, aria_stream_t stream_) {
     if (force == 2) two_cta = d->m > BM;
   }
   int BN;
-  if (d->epilogue == ARIA_EPI_HEADS) {
+  if (epi == ARIA_EPI_HEADS) {
     ARIA_CHECK_ARG(d->head_dim > 0 && d->head_dim % 8 == 0 && d->head_ld >= d->head_dim && d->n % d->head_dim == 0);
     if (d->rope_mask) ARIA_CHECK_ARG(d->head_dim == 128 && d->rope_cos && d->rope_sin);
     if (d->n % 128 == 0) {
@@ -362,7 +368,7 @@ extern "C" int aria_gemm(const aria_gemm_desc_t* d, aria_stream_t stream_) {
     const char* pe = getenv("ARIA_GEMM_PAIR");
     const bool pair_on = pe && pe[0] == '1';
     const bool ok = swiglu ? (d->n % 128 == 0) : (d->n % 256 == 0);
-    if (pair_on && d->group_counts && d->group_mod < 0 && (-d->group_mod) % 2 == 0 && b_mn && ok && d->epilogue != ARIA_EPI_HEADS) {
+    if (pair_on && d->group_counts && d->group_mod < 0 && (-d->group_mod) % 2 == 0 && b_mn && ok && epi != ARIA_EPI_HEADS) {
       two_cta = true;
       BN = 256;
       p.pair = 1;
@@ -385,9 +391,9 @@ extern "C" int aria_gemm(const aria_gemm_desc_t* d, aria_stream_t stream_) {
   // stages each (bytes in flight bound a weight-streaming GEMM); very wide N (lm_head) keeps 128-column tiles.
   int AM = 128;
   static const bool skinny_on = [] { const char* e = getenv("ARIA_GEMM_SKINNY"); return !(e && e[0] == '0'); }();
-  if (skinny_on && !two_cta && !b_mn && d->num_groups == 1 && d->m <= 32 && BN == 128) {
+  if (skinny_on && !xent && !two_cta && !b_mn && d->num_groups == 1 && d->m <= 32 && BN == 128) {
     AM = 32;
-    if (d->epilogue == ARIA_EPI_LINEAR && d->n_seg == 1 && d->n % 32 == 0 && d->n < 16384) BN = 32;
+    if (epi == ARIA_EPI_LINEAR && d->n_seg == 1 && d->n % 32 == 0 && d->n < 16384) BN = 32;
     if (swiglu && d->n % 32 == 0) BN = 64;
   }
 
@@ -425,11 +431,11 @@ extern "C" int aria_gemm(const aria_gemm_desc_t* d, aria_stream_t stream_) {
   if (max_tiles > (1 << 30)) max_tiles = 1 << 30;
 
   if (two_cta)
-    return launch_gemm2_dispatch(BN, b_mn, d->epilogue, tmA, tmB, p, static_cast<int>(max_tiles), stream);
+    return launch_gemm2_dispatch(BN, b_mn, epi, tmA, tmB, p, static_cast<int>(max_tiles), stream);
 
 #define ARIA_LAUNCH(BN_, MN_, EPI_) return launch_gemm<BN_, MN_, EPI_>(tmA, tmB, p, static_cast<int>(max_tiles), stream)
   if (AM == 32) {
-    if (d->epilogue == ARIA_EPI_HEADS) return launch_gemm<128, false, ARIA_EPI_HEADS, 32>(tmA, tmB, p, static_cast<int>(max_tiles), stream);
+    if (epi == ARIA_EPI_HEADS) return launch_gemm<128, false, ARIA_EPI_HEADS, 32>(tmA, tmB, p, static_cast<int>(max_tiles), stream);
     if (swiglu) {
       if (BN == 64) return launch_gemm<64, false, ARIA_EPI_SWIGLU, 32>(tmA, tmB, p, static_cast<int>(max_tiles), stream);
       return launch_gemm<128, false, ARIA_EPI_SWIGLU, 32>(tmA, tmB, p, static_cast<int>(max_tiles), stream);
@@ -437,7 +443,7 @@ extern "C" int aria_gemm(const aria_gemm_desc_t* d, aria_stream_t stream_) {
     if (BN == 32) return launch_gemm<32, false, ARIA_EPI_LINEAR, 32>(tmA, tmB, p, static_cast<int>(max_tiles), stream);
     return launch_gemm<128, false, ARIA_EPI_LINEAR, 32>(tmA, tmB, p, static_cast<int>(max_tiles), stream);
   }
-  if (d->epilogue == ARIA_EPI_HEADS) {
+  if (epi == ARIA_EPI_HEADS) {
     if (BN == 128) ARIA_LAUNCH(128, false, ARIA_EPI_HEADS);
     ARIA_LAUNCH(144, false, ARIA_EPI_HEADS);
   }
@@ -446,10 +452,22 @@ extern "C" int aria_gemm(const aria_gemm_desc_t* d, aria_stream_t stream_) {
     if (b_mn) ARIA_LAUNCH(128, true, ARIA_EPI_SWIGLU);
     ARIA_LAUNCH(128, false, ARIA_EPI_SWIGLU);
   }
+  if (xent) {  // BN = 128 here: the 256-wide tiles only run on CTA pairs
+    if (epi == EPI_XENT_STATS) ARIA_LAUNCH(128, false, EPI_XENT_STATS);
+    if (epi == EPI_XENT_GRAD) ARIA_LAUNCH(128, false, EPI_XENT_GRAD);
+    ARIA_LAUNCH(128, true, EPI_ACC_F32);
+  }
   if (b_mn && BN == 256) ARIA_LAUNCH(256, true, ARIA_EPI_LINEAR);
   if (b_mn) ARIA_LAUNCH(128, true, ARIA_EPI_LINEAR);
   ARIA_LAUNCH(128, false, ARIA_EPI_LINEAR);
 #undef ARIA_LAUNCH
+}
+}  // namespace aria
+
+extern "C" int aria_gemm(const aria_gemm_desc_t* d, aria_stream_t stream) {
+  ARIA_CHECK_ARG(d != nullptr);
+  ARIA_CHECK_ARG(d->epilogue == ARIA_EPI_LINEAR || d->epilogue == ARIA_EPI_SWIGLU || d->epilogue == ARIA_EPI_HEADS);
+  return gemm_run(d, d->epilogue, nullptr, reinterpret_cast<cudaStream_t>(stream));
 }
 
 extern "C" int aria_grouped_gemm(const void* a, const void* b, void* out, const int32_t* group_offsets, int64_t rows,

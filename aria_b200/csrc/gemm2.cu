@@ -234,6 +234,9 @@ static int launch_gemm2(const CUtensorMap& tmA, const CUtensorMap* tmB, const Ge
 int launch_gemm2_dispatch(int bn, bool b_mn, int epi, const CUtensorMap& tmA, const CUtensorMap* tmB, const GemmParams& p,
                           int max_tiles, cudaStream_t stream) {
 #define G2(BN_, MN_, EPI_) return launch_gemm2<BN_, MN_, EPI_>(tmA, tmB, p, max_tiles, stream)
+  if (epi == EPI_XENT_STATS) { if (bn == 256) G2(256, false, EPI_XENT_STATS); G2(128, false, EPI_XENT_STATS); }
+  if (epi == EPI_XENT_GRAD) { if (bn == 256) G2(256, false, EPI_XENT_GRAD); G2(128, false, EPI_XENT_GRAD); }
+  if (epi == EPI_ACC_F32) { if (bn == 256) G2(256, true, EPI_ACC_F32); G2(128, true, EPI_ACC_F32); }
   if (epi == ARIA_EPI_SWIGLU) {
     if (bn == 256) { if (b_mn) G2(256, true, ARIA_EPI_SWIGLU); G2(256, false, ARIA_EPI_SWIGLU); }
     if (b_mn) G2(128, true, ARIA_EPI_SWIGLU);

@@ -25,6 +25,29 @@ constexpr int A_STAGE_BYTES = BM * BK * 2;  // 16 KB
 constexpr int GEMM_THREADS = 320;  // warp 0 TMA, warp 1 MMA, warps 2-9 epilogue (two warps per TMEM lane quadrant)
 constexpr int EPI_WARPS = 8;
 
+// Internal epilogues of the fused lm_head + cross-entropy (lm_loss.cu); never accepted by aria_gemm.
+//   XENT_STATS: z = bf16(acc), columns >= V are -inf; per row, one (max, sum exp(z - max)) partial per 64 columns, and the
+//               target's logit
+//   XENT_GRAD : out = bf16((exp(z - lse[r]) - [v0 + c == target[r]]) * dloss / n_valid), 0 for ignored rows
+//   ACC_F32   : acc32 = acc (+ acc32 unless first); the last call stores bf16(acc32) to out instead
+constexpr int EPI_XENT_STATS = 3;
+constexpr int EPI_XENT_GRAD = 4;
+constexpr int EPI_ACC_F32 = 5;
+constexpr int XENT_SLOT = 64;  // columns per (max, sum) partial
+
+struct XentParams {
+  const int32_t* target;   // [M], < 0: ignored row
+  const float* lse;        // [M] natural log (GRAD)
+  float2* part;            // [ceil(V / 64)][M] (STATS)
+  float* tlogit;           // [M] (STATS)
+  const float* dloss;      // [1] (GRAD)
+  const int32_t* n_valid;  // [1] (GRAD)
+  float* acc;              // [M, N] fp32 (ACC_F32)
+  int64_t M;
+  int V, v0;               // vocabulary size; global column of the tile's column 0 (GRAD)
+  int first, last;         // ACC_F32
+};
+
 struct GemmParams {
   int M, N, K;  // N = output columns per segment
   int num_groups;
@@ -50,6 +73,7 @@ struct GemmParams {
   const __nv_bfloat16* rope_sin;
   const int32_t* position_ids;
   int dbg_lbo, dbg_sbo, dbg_kadv;
+  XentParams x;
 };
 
 ARIA_DEVICE int weight_block(const GemmParams& p, int grp) {
@@ -178,6 +202,107 @@ ARIA_DEVICE void epilogue_tile(const GemmParams& p, const uint32_t taddr, const 
           const int col = n_idx * OUT_BN + c + q * 8;
           if (col + 8 <= p.N)
             *reinterpret_cast<uint4*>(orow + c + q * 8) = make_uint4(o[q * 4], o[q * 4 + 1], o[q * 4 + 2], o[q * 4 + 3]);
+        }
+      }
+    }
+  } else if constexpr (EPI == EPI_XENT_STATS) {
+    // log-sum-exp partials of the bf16-rounded logits; this warp's half of the tile is 1 (BN = 128) or 2 (BN = 256) slots
+    constexpr float L2E = 1.4426950408889634f;
+    const int col0 = n_idx * BN + half * (BN / 2);
+    const int t = row_ok ? p.x.target[grow] : -1;
+    float m = -INFINITY, s = 0.f;
+#pragma unroll 1
+    for (int c = 0; c < BN / 2; c += 32) {
+      uint32_t v[32];
+      tmem_ld_32x32(taddr + half * (BN / 2) + c, v);
+      tmem_ld_wait();
+      const int cb = col0 + c;
+      float z[32], cm = -INFINITY, zt = 0.f;
+#pragma unroll
+      for (int j = 0; j < 32; ++j) {
+        z[j] = cb + j < p.x.V ? bf16r(__uint_as_float(v[j])) : -INFINITY;
+        cm = fmaxf(cm, z[j]);
+        if (cb + j == t) zt = z[j];
+      }
+      if (row_ok && t >= cb && t < cb + 32) p.x.tlogit[grow] = zt;
+      if (cm > -INFINITY) {
+        const float mn = fmaxf(m, cm);
+        float a = 0.f;
+#pragma unroll
+        for (int j = 0; j < 32; ++j) a += exp2f((z[j] - mn) * L2E);
+        s = s * exp2f((m - mn) * L2E) + a;
+        m = mn;
+      }
+      if ((c & (XENT_SLOT - 1)) == XENT_SLOT - 32) {  // end of a 64-column slot
+        const int slot0 = cb + 32 - XENT_SLOT;
+        if (row_ok && slot0 < p.x.V) p.x.part[static_cast<int64_t>(slot0 / XENT_SLOT) * p.x.M + grow] = make_float2(m, s);
+        m = -INFINITY;
+        s = 0.f;
+      }
+    }
+  } else if constexpr (EPI == EPI_XENT_GRAD) {
+    // d loss / d z of one vocabulary chunk (tile columns are chunk columns; global column = v0 + chunk column)
+    constexpr float L2E = 1.4426950408889634f;
+    const int col0 = n_idx * BN;
+    int t = -1;
+    float lse = 0.f;
+    if (row_ok) {
+      t = p.x.target[grow];
+      lse = p.x.lse[grow];
+    }
+    const int nv = *p.x.n_valid;
+    const float scale = (t >= 0 && nv > 0) ? *p.x.dloss / static_cast<float>(nv) : 0.f;
+    const int tc = t - p.x.v0;  // target as a chunk column
+    __nv_bfloat16* orow = p.out[0] + grow * p.ldo;
+#pragma unroll 1
+    for (int c = half * (BN / 2); c < (half + 1) * (BN / 2); c += 32) {
+      uint32_t v[32];
+      tmem_ld_32x32(taddr + c, v);
+      tmem_ld_wait();
+      if (!row_ok) continue;
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        const int col = col0 + c + q * 8;
+        if (col + 8 > p.N) continue;
+        float g[8];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          const float z = bf16r(__uint_as_float(v[q * 8 + j]));
+          g[j] = (exp2f((z - lse) * L2E) - (col + j == tc ? 1.f : 0.f)) * scale;
+        }
+        *reinterpret_cast<uint4*>(orow + col) =
+            make_uint4(pack_bf16(g[0], g[1]), pack_bf16(g[2], g[3]), pack_bf16(g[4], g[5]), pack_bf16(g[6], g[7]));
+      }
+    }
+  } else if constexpr (EPI == EPI_ACC_F32) {
+    const int col0 = n_idx * BN;
+    float* arow = p.x.acc + grow * p.N;
+    __nv_bfloat16* orow = p.out[0] + grow * p.ldo;
+#pragma unroll 1
+    for (int c = half * (BN / 2); c < (half + 1) * (BN / 2); c += 32) {
+      uint32_t v[32];
+      tmem_ld_32x32(taddr + c, v);
+      tmem_ld_wait();
+      if (!row_ok) continue;
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        const int col = col0 + c + q * 8;
+        if (col + 8 > p.N) continue;
+        float x[8];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) x[j] = __uint_as_float(v[q * 8 + j]);
+        float4* a4 = reinterpret_cast<float4*>(arow + col);
+        if (!p.x.first) {
+          const float4 u = a4[0], w = a4[1];
+          x[0] += u.x; x[1] += u.y; x[2] += u.z; x[3] += u.w;
+          x[4] += w.x; x[5] += w.y; x[6] += w.z; x[7] += w.w;
+        }
+        if (p.x.last) {
+          *reinterpret_cast<uint4*>(orow + col) =
+              make_uint4(pack_bf16(x[0], x[1]), pack_bf16(x[2], x[3]), pack_bf16(x[4], x[5]), pack_bf16(x[6], x[7]));
+        } else {
+          a4[0] = make_float4(x[0], x[1], x[2], x[3]);
+          a4[1] = make_float4(x[4], x[5], x[6], x[7]);
         }
       }
     }

@@ -17,6 +17,7 @@ from __future__ import annotations
 from typing import Optional
 
 import torch
+import torch.utils.checkpoint
 
 from . import ops
 from .moe_train import moe_layer_train
@@ -142,3 +143,104 @@ def decoder_layer_train(layer, hidden_states: torch.Tensor, position_ids: Option
                                 attn.num_heads, rope, key_mask, pos)
     h, x = RMSNormFunction.apply(x, layer.post_attention_layernorm.weight, eps2)
     return ResidualAddFunction.apply(moe_layer_train(layer.mlp, h, router_losses), x)
+
+
+# ------------------------------------------------------------------------------------------------ whole language model
+class EmbeddingFunction(torch.autograd.Function):
+    """nn.Embedding on aria_embedding; the backward (aria_embedding_bwd, only when the table requires grad) sums the rows per
+    id in position order.  Positions whose id is skip_id get no gradient: they are image tokens, whose embeddings the image
+    features replaced (masked_scatter, modeling_aria.py:272-283)."""
+
+    @staticmethod
+    def forward(ctx, ids, table, skip_id: Optional[int] = None):
+        ids = ids.contiguous()
+        ctx.save_for_backward(ids)
+        ctx.vocab, ctx.skip_id = table.shape[0], skip_id
+        return ops.embedding(ids, table)
+
+    @staticmethod
+    def backward(ctx, g):
+        if not ctx.needs_input_grad[1]:
+            return None, None, None
+        (ids,) = ctx.saved_tensors
+        return None, ops.embedding_bwd(ids, g.contiguous(), ctx.vocab, ctx.skip_id), None
+
+
+class _MergeImageFunction(torch.autograd.Function):
+    """embeds with the image-token rows replaced by the (constant) image features; the gradient passes through unchanged (the
+    embedding backward skips the image-token rows)."""
+
+    @staticmethod
+    def forward(ctx, embeds, ids, image_token: int, features):
+        out = embeds.clone()
+        ops.merge_image_features(ids.reshape(-1).contiguous(), image_token, features.reshape(-1, features.shape[-1]),
+                                 out.view(-1, out.shape[-1]))
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        return g, None, None, None
+
+
+class LMHeadCrossEntropyFunction(torch.autograd.Function):
+    """(h [M, d], w [V, d], targets [M] int32, < 0 = ignored) -> mean cross-entropy of the bf16 logits h w^T over the valid rows,
+    a 0-dim fp32 tensor, through the fused kernels (aria_lm_xent_fwd / _bwd): no [M, V] tensor is ever allocated.  The
+    lm_head gradient is skipped when w does not require grad."""
+
+    @staticmethod
+    def forward(ctx, h, w, targets):
+        loss, lse, n_valid = ops.lm_xent_fwd(h, w, targets)
+        ctx.save_for_backward(h, w, targets, lse, n_valid)
+        return loss
+
+    @staticmethod
+    def backward(ctx, dloss):
+        h, w, targets, lse, n_valid = ctx.saved_tensors
+        dh, dw = ops.lm_xent_bwd(h, w, targets, lse, n_valid, dloss, need_dw=ctx.needs_input_grad[1])
+        return (dh if ctx.needs_input_grad[0] else None), dw, None
+
+
+def shifted_targets(labels: torch.Tensor, attention_mask: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """int32 [B*T] targets of the shifted loss (modeling_aria.py:300-323): position t of row b predicts labels[b, t+1]; it is
+    ignored (-1) when attention_mask[b, t+1] == 0, when that label is negative (ignore_index -100) and at the last position.
+    Index plumbing on the labels' device, no sync."""
+    B, T = labels.shape
+    tgt = torch.full((B, T), -1, dtype=torch.int32, device=labels.device)
+    if T > 1:
+        nxt = labels[:, 1:]
+        keep = nxt >= 0
+        if attention_mask is not None:
+            keep = keep & (attention_mask[:, -(T - 1):].to(labels.device) != 0)
+        tgt[:, :-1] = torch.where(keep, nxt, torch.full_like(nxt, -1)).to(torch.int32)
+    return tgt.reshape(-1)
+
+
+def causal_lm_loss(lm, labels: torch.Tensor, input_ids: Optional[torch.Tensor] = None, inputs_embeds: Optional[torch.Tensor] = None,
+                   attention_mask: Optional[torch.Tensor] = None, position_ids: Optional[torch.Tensor] = None,
+                   router_losses: bool = False, gradient_checkpointing: bool = False,
+                   skip_embed_id: Optional[int] = None) -> torch.Tensor:
+    """Training loss of an `aria_b200.moe_lm.AriaMoELMForCausalLM` with a grad_fn: embedding -> every decoder layer
+    (decoder_layer_train) -> final RMSNorm -> fused lm_head + shifted cross-entropy (the loss of modeling_aria.py:300-323).
+    input_ids [B, T] (embedded here; positions whose id is skip_embed_id get no embedding gradient) or inputs_embeds [B, T, d];
+    labels [B, T]; attention_mask: the HF 2-D padding mask, 1 = keep; position_ids [B, T] (default: arange per row).
+    gradient_checkpointing=True keeps only each layer's input and recomputes the layer in backward
+    (torch.utils.checkpoint, use_reentrant=False); every kernel and the routing are deterministic, so the recompute
+    reproduces the forward bit for bit."""
+    model = lm.model
+    if inputs_embeds is None:
+        x = EmbeddingFunction.apply(input_ids, model.embed_tokens.weight, skip_embed_id)
+    else:
+        x = inputs_embeds
+    dev = x.device
+    if attention_mask is not None:
+        attention_mask = attention_mask.to(dev)
+    for layer in model.layers:
+        if gradient_checkpointing:
+            x = torch.utils.checkpoint.checkpoint(decoder_layer_train, layer, x, position_ids, attention_mask, router_losses,
+                                                  use_reentrant=False)
+        else:
+            x = decoder_layer_train(layer, x, position_ids, attention_mask, router_losses)
+    h, _ = RMSNormFunction.apply(x, model.norm.weight, model.norm.variance_epsilon)
+    d = h.shape[-1]
+    targets = shifted_targets(labels.to(dev), attention_mask)
+    return LMHeadCrossEntropyFunction.apply(h.reshape(-1, d), lm.lm_head.weight, targets)

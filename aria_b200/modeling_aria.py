@@ -191,6 +191,38 @@ class AriaForConditionalGeneration(nn.Module):
             out.loss = self._shifted_cross_entropy(logits, labels, attention_mask)
         return out
 
+    def training_loss(self, input_ids: torch.Tensor, labels: torch.Tensor, pixel_values: Optional[torch.Tensor] = None,
+                      pixel_mask: Optional[torch.Tensor] = None, attention_mask: Optional[torch.Tensor] = None,
+                      position_ids: Optional[torch.Tensor] = None, router_losses: bool = False,
+                      gradient_checkpointing: bool = False) -> torch.Tensor:
+        """The loss of forward(..., labels=labels) as a tensor with a grad_fn, for fine-tuning the language model (the recipes'
+        freeze_vit; aria_b200.lm_train.causal_lm_loss does the work).  The vision tower and projector run without grad and
+        their features replace the image-token embeddings as in forward(); the image-token row of the embedding table gets no
+        gradient.  Their backward is not built: a vision-tower or projector parameter that requires grad raises
+        NotImplementedError (call freeze_vit() / freeze_projector())."""
+        from .lm_train import _MergeImageFunction, causal_lm_loss
+        if any(p.requires_grad for m in (self.vision_tower, self.multi_modal_projector) for p in m.parameters()):
+            raise NotImplementedError("aria_b200: the vision tower / projector backward is not implemented; freeze them "
+                                      "(freeze_vit(), freeze_projector()) to train the language model")
+        dev = self.device
+        input_ids = input_ids.to(dev)
+        lm = self.language_model
+        embeds = None
+        if pixel_values is not None:
+            from .lm_train import EmbeddingFunction
+            with torch.no_grad():
+                feats, image_attn_mask = self.vision_tower(pixel_values.to(dev, bf16), pixel_mask)
+                image_features = self.multi_modal_projector(feats, image_attn_mask)
+            n_image_tokens = int((input_ids == self.config.image_token_index).sum())
+            if n_image_tokens != image_features.shape[0] * image_features.shape[1]:
+                raise ValueError(f"Image features and image tokens do not match: tokens: {n_image_tokens}, "
+                                 f"features {image_features.shape[0] * image_features.shape[1]}")
+            embeds = EmbeddingFunction.apply(input_ids, lm.model.embed_tokens.weight, self.config.image_token_index)
+            embeds = _MergeImageFunction.apply(embeds, input_ids, self.config.image_token_index, image_features)
+        return causal_lm_loss(lm, labels, input_ids=None if embeds is not None else input_ids, inputs_embeds=embeds,
+                              attention_mask=attention_mask, position_ids=position_ids, router_losses=router_losses,
+                              gradient_checkpointing=gradient_checkpointing, skip_embed_id=self.config.image_token_index)
+
     @staticmethod
     def _shifted_cross_entropy(logits, labels, attention_mask):
         """modeling_aria.py:300-323, verbatim semantics: tokens < n predict n; padded positions dropped through the 2-D mask."""

@@ -542,6 +542,64 @@ def embedding(ids: torch.Tensor, table: torch.Tensor) -> torch.Tensor:
     return out
 
 
+def embedding_bwd(ids: torch.Tensor, dout: torch.Tensor, vocab: int, skip_id: Optional[int] = None) -> torch.Tensor:
+    """Gradient of `embedding(ids, table)` w.r.t. a [vocab, d] table: rows summed per id in fp32, in position order (bit-
+    reproducible); positions with id == skip_id and out-of-range ids contribute nothing; rows no position uses are zero."""
+    _chk(ids, torch.int64, align=8), _chk(dout)
+    d = dout.shape[-1]
+    n = ids.numel()
+    assert dout.numel() == n * d
+    dtable = torch.zeros((vocab, d), dtype=bf16, device=dout.device)
+    lib = L.load()
+    nbytes = lib.aria_embedding_bwd_workspace_bytes(n, vocab)
+    ws = torch.empty((nbytes,), dtype=torch.uint8, device=dout.device)
+    with torch.cuda.device(dout.device):
+        L.check(lib.aria_embedding_bwd(_p(ids), _p(dout), _p(dtable), n, d, vocab, -1 if skip_id is None else int(skip_id), _p(ws),
+                                       nbytes, _stream(dout)), "embedding_bwd")
+    return dtable
+
+
+def lm_xent_fwd(h: torch.Tensor, w: torch.Tensor, target: torch.Tensor):
+    """Fused lm_head + cross-entropy: h [M, d] bf16, w [V, d] (nn.Linear layout), target [M] int32 (< 0: ignored)
+    -> (loss 0-dim fp32 = mean over valid rows, lse [M] fp32 (natural log), n_valid [1] int32).  No [M, V] tensor exists."""
+    _chk(h), _chk(w), _chk(target, torch.int32, align=4)
+    M, d = h.shape
+    V = w.shape[0]
+    assert w.shape[1] == d and target.numel() == M
+    dev = h.device
+    lse = torch.empty((M,), dtype=torch.float32, device=dev)
+    loss = torch.full((1,), float("nan"), dtype=torch.float32, device=dev)
+    n_valid = torch.zeros((1,), dtype=torch.int32, device=dev)
+    lib = L.load()
+    nbytes = lib.aria_lm_xent_fwd_workspace_bytes(M, V)
+    ws = torch.empty((max(nbytes, 16),), dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        L.check(lib.aria_lm_xent_fwd(_p(h), _p(w), _p(target), _p(lse), _p(loss), _p(n_valid), M, V, d, _p(ws), ws.numel(),
+                                     _stream(h)), "lm_xent_fwd")
+    return loss.view(()), lse, n_valid
+
+
+def lm_xent_bwd(h: torch.Tensor, w: torch.Tensor, target: torch.Tensor, lse: torch.Tensor, n_valid: torch.Tensor,
+                dloss: torch.Tensor, need_dw: bool = True, workspace_bytes: Optional[int] = None):
+    """Backward of `lm_xent_fwd` for the upstream gradient dloss (1-element fp32 tensor, read on the device)
+    -> (dh [M, d], dw [V, d] or None).  workspace_bytes: size of the chunk workspace (default: the library's, a 512 MiB
+    chunk budget); a smaller one walks the vocabulary in more chunks."""
+    _chk(h), _chk(w), _chk(target, torch.int32, align=4), _chk(lse, torch.float32), _chk(n_valid, torch.int32, align=4)
+    dloss = dloss.reshape(1).to(torch.float32).contiguous()
+    M, d = h.shape
+    V = w.shape[0]
+    dev = h.device
+    dh = torch.empty_like(h)
+    dw = torch.empty_like(w) if need_dw else None
+    lib = L.load()
+    nbytes = lib.aria_lm_xent_bwd_workspace_bytes(M, V, d) if workspace_bytes is None else int(workspace_bytes)
+    ws = torch.empty((max(nbytes, 16),), dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        L.check(lib.aria_lm_xent_bwd(_p(h), _p(w), _p(target), _p(lse), _p(n_valid), _p(dloss), _p(dh), _p(dw), M, V, d, _p(ws),
+                                     nbytes, _stream(h)), "lm_xent_bwd")
+    return dh, dw
+
+
 def merge_image_features(ids: torch.Tensor, image_token: int, features: torch.Tensor, embeds: torch.Tensor,
                          count_out: Optional[torch.Tensor] = None):
     """In place: embeds rows at <|img|> positions <- consecutive rows of features (masked_scatter)."""

@@ -212,6 +212,15 @@ int aria_rmsnorm_bwd(const void* x, const void* weight, const void* dy, const vo
  * tables from aria_rope_table. */
 int aria_rope_bwd(void* x, const void* cos, const void* sin, const int32_t* position_ids, int64_t rows, int32_t n_heads,
                   int32_t rows_per_batch, aria_stream_t stream);
+/* Backward of aria_embedding (autograd of nn.Embedding, moe_lm.py:605-636):  dtable[id] = bf16(sum of dout[p] over the
+ * positions p with ids[p] == id), summed in fp32 in position order.  Positions whose id equals skip_id (< 0: none; the image
+ * token, whose embedding masked_scatter replaced, modeling_aria.py:272-283) and out-of-range ids contribute nothing.  Only
+ * rows that occur are written: the caller zero-fills dtable.  Bit-reproducible (stable counting sort, no atomics on values).
+ * ids [n] int64, dout [n, d] bf16 (d % 8 == 0, d <= 4096), dtable [vocab, d] bf16.
+ * workspace: aria_embedding_bwd_workspace_bytes(n, vocab), 16-byte aligned. */
+int64_t aria_embedding_bwd_workspace_bytes(int64_t n, int64_t vocab);
+int aria_embedding_bwd(const int64_t* ids, const void* dout, void* dtable, int64_t n, int32_t d, int64_t vocab, int64_t skip_id,
+                       void* workspace, int64_t workspace_bytes, aria_stream_t stream);
 /* nn.LayerNorm (Idefics2 encoder layers, projector): out = bf16((x-mean)*rstd*w + b). */
 int aria_layernorm(const void* x, const void* weight, const void* bias, void* out, int64_t rows, int32_t d,
                    float eps, aria_stream_t stream);
@@ -304,6 +313,30 @@ int aria_attention_bwd(const void* q, const void* k, const void* v, const void* 
                        void* dk, void* dv, const uint8_t* key_mask, int32_t B, int32_t H, int32_t T, int64_t q_stride_b,
                        int64_t q_stride_h, int64_t kv_stride_b, int64_t kv_stride_h, float scale, int32_t head_dim, int32_t causal,
                        void* workspace, int64_t workspace_bytes, aria_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * Fused lm_head + cross-entropy (training).  Replaces lm_head(h).float() -> nn.CrossEntropyLoss (modeling_aria.py:300-323)
+ * and its autograd without materialising the [M, V] logits.
+ *   h [M, d] bf16 (final-norm output, one row per predicting position), w [V, d] bf16 (nn.Linear layout),
+ *   target [M] int32: the class of each row, < 0 = ignored (ignore_index, padding, last position).  A target >= V does not
+ *   fault; it makes the loss NaN.  Logits are the bf16-rounded GEMM outputs, as the reference's bf16 lm_head returns them.
+ * ------------------------------------------------------------------------------------------------ */
+/* Forward: lse [M] fp32 (natural log, every row), loss [1] = mean over valid rows of lse - z_target (NaN with no valid row),
+ * n_valid [1] = number of rows with target >= 0.  Deterministic (fixed-order reductions), no host sync.
+ * d % 8 == 0, V % 8 == 0; M = 0 does nothing.  workspace: aria_lm_xent_fwd_workspace_bytes(M, V), 16-byte aligned. */
+int64_t aria_lm_xent_fwd_workspace_bytes(int64_t M, int64_t V);
+int aria_lm_xent_fwd(const void* h, const void* w, const int32_t* target, float* lse, float* loss, int32_t* n_valid, int64_t M,
+                     int64_t V, int32_t d, void* workspace, int64_t workspace_bytes, aria_stream_t stream);
+/* Backward for the upstream gradient dloss [1] (device): with g = (softmax(z) - onehot(target)) * dloss / n_valid (0 for ignored
+ * rows), dh [M, d] = g @ w (accumulated in fp32, rounded once) and dw [V, d] = g^T h (NULL: lm_head frozen, not computed).
+ * The vocabulary is walked in chunks of Vc columns (a multiple of 256: the largest whose bf16 [M, Vc] buffer fits the
+ * workspace after its fixed part M*d*4 + 256 bytes, at least 256); aria_lm_xent_bwd_workspace_bytes returns the default,
+ * a 512 MiB chunk budget (or the whole vocabulary if smaller).  dloss and n_valid are read on the device, so the call
+ * can be captured in a CUDA graph.  Deterministic.  d % 64 == 0, V % 8 == 0; M = 0 does nothing. */
+int64_t aria_lm_xent_bwd_workspace_bytes(int64_t M, int64_t V, int32_t d);
+int aria_lm_xent_bwd(const void* h, const void* w, const int32_t* target, const float* lse, const int32_t* n_valid,
+                     const float* dloss, void* dh, void* dw /* NULL: lm_head frozen */, int64_t M, int64_t V, int32_t d,
+                     void* workspace, int64_t workspace_bytes, aria_stream_t stream);
 
 #ifdef __cplusplus
 }
